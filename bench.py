@@ -2,6 +2,7 @@
 """bench.py -- plan-loop Hz / rollout-steps per second of the MPPI rollout hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c2|c3|c4|c5] [--scaling strong|weak]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE MPPI plan of a BASELINE configuration: shift U -> K1 sample/clamp -> K2 articulated rollout -> Objective cost ->
@@ -19,6 +20,8 @@ Printed JSON (rank 0, one line):
   roofline      K3 (fused cost-softmax-weighted-sum) achieved HBM GB/s vs the measured peak (MEASURED_PEAKS.json)
   cpu_baseline  the CPU restatement of the reference pipeline (oracle/) on this box's host cores (N = 1 only), with its parallel efficiency
   correctness   N > 1: max |action| difference across ranks and between the peer-memory exchange and the NCCL all-gather
+--dump-outputs DIR writes what the last timed plan returned to its caller as DIR/<name>.npy (rank 0, see dump_outputs); the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 --impl reference times that CPU restatement as the reference arm (the reference's own engines, IsaacGym/PhysX and mppi_torch, are
 closed / un-vendored and cannot run here: BASELINE.md section 2).
 """
@@ -30,6 +33,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True         # the tree may be read-only; bench.py leaves nothing in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -423,6 +427,20 @@ def timed_plans(planner, steps, warmup, flush, barrier, clocks=None):
     return [s.elapsed_time(e) for s, e in zip(starts, ends)]
 
 
+def dump_outputs(planner, out_dir, n_samples=4096):
+    """float32 .npy files of what the last plan handed its caller: `action` (the first action, command()'s return value),
+    `mean_action` (the updated control sequence U, (T, nu)) and `perturbed_action_sample` (the sampled control sequences of a fixed
+    seeded subset of at most `n_samples` of the K samples, in ascending sample order, (n, T, nu)) -- under 6 MB at every configuration."""
+    m = planner.mppi
+    torch.cuda.synchronize()
+    idx = np.sort(np.random.default_rng(0).choice(m.K, min(m.K, n_samples), replace=False))
+    outs = {"action": m._action, "mean_action": m.mean_action,
+            "perturbed_action_sample": m.perturbed_action[torch.as_tensor(idx, device=m.actions.device)]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to(torch.float32).cpu().numpy())
+
+
 def run_gpu_arm(args, rank, world, local_rank):
     import torch.distributed as dist
     import __graft_entry__
@@ -458,6 +476,8 @@ def run_gpu_arm(args, rank, world, local_rank):
 
     # ---- device-resident timing ------------------------------------------------------------------------------------
     per_step_ms = timed_plans(planner, args.steps, args.warmup, flush, barrier, clocks)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(planner, args.dump_outputs)
     graph_on = planner.mppi._graph is not None
     total_s = reduce_max(sum(per_step_ms)) * 1e-3
     value = k_total * T * args.steps / total_s
@@ -644,7 +664,12 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed plan's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm: the reference arm picks its sample count from the host's speed")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -8,15 +8,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
-REFERENCE = "/root/reference"          # exists only in the build container, never on the GPU box
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-
-
-def has_reference():
-    return os.path.isdir(os.path.join(REFERENCE, "assets", "urdf"))
 
 
 @pytest.fixture(scope="session")

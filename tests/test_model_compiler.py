@@ -1,13 +1,13 @@
 """URDF -> model-constants compiler: pinned against forward kinematics computed straight from the reference URDFs by
 an independent homogeneous-transform walk (tests/golden/fk_reference_urdf.json, made by make_golden.py), the
-known answers of SURVEY.md Appendix B, and -- in the build container only -- a re-compile from /root/reference."""
+known answers of SURVEY.md Appendix B, and the reference's own example configs and compiled URDFs
+(tests/golden/reference_examples.json, made by make_reference_examples.py)."""
 import json
 import os
 
 import numpy as np
 import pytest
 
-from conftest import REFERENCE, has_reference
 from mppi_isaac_b200.model.blob import compiled_path, build_scene
 from mppi_isaac_b200.model.urdf import (compile_urdf, forward_kinematics, load_compiled, mesh_inertia, quat_xyzw_to_R)
 from mppi_isaac_b200.utils.config_store import load_actor_cfgs, load_config, load_isaacgym_config
@@ -93,34 +93,39 @@ def test_config_loader_builtin_and_errors(tmp_path):
         load_config(str(f))
 
 
-@pytest.mark.skipif(not has_reference(), reason="reference checkout only exists in the build container")
-def test_reference_configs_and_urdfs_load_unchanged():
+def test_reference_configs_and_urdfs_load_unchanged(tmp_path):
     import glob
-    conf = [os.path.join(REFERENCE, "conf")]
-    tasks = sorted(glob.glob(os.path.join(REFERENCE, "examples", "*", "*.yaml")))
+    with open(os.path.join(GOLD, "reference_examples.json")) as f:
+        gold = json.load(f)
+    for rel, text in gold["files"].items():                       # the reference's conf/ and examples/ YAMLs, verbatim
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(text)
+    conf = [str(tmp_path / "conf")]
+    tasks = sorted(glob.glob(str(tmp_path / "examples" / "*" / "*.yaml")))
     assert len(tasks) >= 10
     for t in tasks:
         cfg = load_config(t, conf)
         assert cfg.mppi.num_samples > 0 and len(cfg.actors) > 0
-    for rel in ("point_robot.urdf", "heijn/heijn.urdf", "panda_isaac/robots/franka_panda_stick.urdf"):
-        fresh = compile_urdf(os.path.join(REFERENCE, "assets", "urdf", rel))
+    for rel, fresh in gold["urdf"].items():                        # compiled from the reference's assets/
         shipped = load_compiled(compiled_path(rel))
-        np.testing.assert_allclose(fresh.mass, shipped.mass, rtol=1e-12)
-        np.testing.assert_allclose(fresh.inertia_o, shipped.inertia_o, rtol=1e-9, atol=1e-12)
-        assert fresh.link_names == shipped.link_names and fresh.dof_names == shipped.dof_names
-    # every example scene of the reference builds from ITS conf/ and assets/ (anymal: legged floating base, out of scope)
+        np.testing.assert_allclose(fresh["mass"], shipped.mass, rtol=1e-12)
+        np.testing.assert_allclose(fresh["inertia_o"], shipped.inertia_o, rtol=1e-9, atol=1e-12)
+        assert fresh["link_names"] == shipped.link_names and fresh["dof_names"] == shipped.dof_names
+    # every example scene of the reference builds from ITS conf/ on the shipped models_compiled/ into the scene its own assets/ gave
+    # (anymal: legged floating base, out of scope)
     built = {}
     for t in tasks:
         cfg = load_config(t, conf)
         name = os.path.basename(os.path.dirname(t))
         try:
-            sc = build_scene(load_actor_cfgs(cfg.actors, conf), assets_dirs=[os.path.join(REFERENCE, "assets")], substep=cfg.isaacgym.dt / cfg.isaacgym.substeps)
-            built[name] = (sc.model.nb, sc.nu)
-        except NotImplementedError as e:
-            built[name] = str(e)
-    assert isinstance(built.pop("anymal"), str)
-    assert all(isinstance(v, tuple) for v in built.values()), built
-    assert built["albert"] == (12, 9) and built["omni_panda_pick"] == (12, 12) and built["panda_effort"] == (7, 7) and built["panda_stick_push"][0] == 7
+            sc = build_scene(load_actor_cfgs(cfg.actors, conf), substep=cfg.isaacgym.dt / cfg.isaacgym.substeps)
+            built[name] = [sc.model.nb, sc.nu, sc.model.nlinks, sc.num_bodies]
+        except NotImplementedError:
+            built[name] = "NotImplementedError"
+    assert built == gold["scenes"]
+    assert built.pop("anymal") == "NotImplementedError"
+    assert all(isinstance(v, list) for v in built.values()), built
+    assert built["albert"][:2] == [12, 9] and built["omni_panda_pick"][:2] == [12, 12] and built["panda_effort"][:2] == [7, 7] and built["panda_stick_push"][0] == 7
     a = load_actor_cfgs(["panda_stick", "goal"], conf)
     b = load_actor_cfgs(["panda_stick", "goal"])
     assert a[0].urdf_file == b[0].urdf_file and a[0].init_joint_pose == b[0].init_joint_pose and a[1].init_pos == b[1].init_pos
